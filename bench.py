@@ -31,6 +31,14 @@ clocks/throttle reasons are sampled during the timed region.
 ``e2e`` repeats the measurement (at most 6 timed steps) through the public training API (`pretrain.forward_backward_pass` /
 `take_optimizer_step`) with every micro-batch copied from pinned host memory inside the timed region and
 the loss read back to the host every optimizer step.
+
+``--dump-outputs DIR`` (this repository's arm, the config chosen on the command line) writes what the last timed step computed, after the
+timing: ``DIR/loss.npy`` (float32, the loss of each micro-batch as ``forward_backward_pass`` returned it) and
+``DIR/params_sample.npy`` (float32, the fp32 master weights after the LAMB update at DUMP_SAMPLE positions drawn
+from a fixed seed).  Inputs, initial weights and dropout masks follow ``--seed``, so two builds run with the same
+arguments can be compared output by output.  Compare with a tolerance: the gradient reductions are not bitwise
+reproducible, and two runs of one build differed by up to 1.5e-5 in a micro-batch loss (~0.13) and 3e-6 in a sampled
+weight (NVIDIA B200 at a 1000 W power limit, phase 1, 4 timed steps).
 """
 from __future__ import annotations
 
@@ -56,6 +64,7 @@ ROBERTA = dict(seq=512, local_batch=16, max_pred=80, lr=4e-4, warmup=0.06, max_s
                vocab_size=28996, next_sentence=False, mask_prob=0.15, lr_decay="linear")
 MODEL = dict(vocab_size=30522, hidden_size=1024, num_hidden_layers=24, num_attention_heads=16,
              intermediate_size=4096, max_position_embeddings=512, type_vocab_size=2)
+DUMP_SAMPLE = 1 << 22            # weights kept by --dump-outputs: 16 MB of float32
 
 
 def parse():
@@ -79,6 +88,8 @@ def parse():
                     help="RoBERTa-style recipe (seq 512, no NSP, cased vocabulary, linear decay) instead of --phase; ours only")
     ap.add_argument("--kfac", action="store_true", help="K-FAC preconditioner on (BASELINE config #5); ours only")
     ap.add_argument("--seed", type=int, default=42)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's losses and a fixed sample of the updated weights as DIR/*.npy")
     return ap.parse_args()
 
 
@@ -141,6 +152,18 @@ def timed_steps(run_step, K, W, flusher, dev):
     torch.cuda.synchronize()
     clocks = sampler.stop()
     return e0.elapsed_time(e1) / K, clocks
+
+
+def dump_outputs(out_dir, losses, flat_param):
+    """The last timed step's outputs as float32 .npy files (see the module docstring)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = flat_param.numel()
+    idx = np.sort(np.random.default_rng(1234).choice(n, min(n, DUMP_SAMPLE), replace=False))
+    sample = flat_param[torch.from_numpy(idx).to(flat_param.device)]
+    np.save(os.path.join(out_dir, "loss.npy"), torch.stack(losses).float().cpu().numpy())
+    np.save(os.path.join(out_dir, "params_sample.npy"), sample.float().cpu().numpy())
 
 
 def max_over_ranks(x, dev):
@@ -259,13 +282,16 @@ def run_ours(args, ph, B, accum, rank, world, dev):
     loss_acc = torch.zeros((), device=dev)
 
     opt_events = []
+    step_losses = []                   # the micro-batch losses of the latest step (device tensors, no sync)
 
     def step_device(i):
+        step_losses.clear()
         for m in range(accum):
             batch = dev_pool[(i * accum + m) % len(dev_pool)]
             loss = pretrain.forward_backward_pass(ddp, crit, scaler, batch, accum, sync_grads=(m == accum - 1),
                                                   compute_dtype=torch.bfloat16)
             loss_acc.add_(loss)
+            step_losses.append(loss.detach())
         for sc in scheds:
             sc.step()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -294,6 +320,8 @@ def run_ours(args, ph, B, accum, rank, world, dev):
         parity = fused_parity(comm, arena, opt, dev, rank, world)     # before anything is timed
     l0 = K.KERNEL_LAUNCHES
     ms, clocks = timed_steps(step_device, args.steps, args.warmup, flusher, dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_losses, arena.flat_param)
     timeline = None
     if world > 1 and hasattr(comm, "timeline") and precond is None:
         torch.cuda.synchronize()
@@ -512,6 +540,8 @@ def main():
     if not torch.cuda.is_available():
         print(json.dumps({"impl": args.impl, "unavailable": "no CUDA device"}))
         return
+    if args.dump_outputs and args.impl != "ours":
+        sys.exit("--dump-outputs dumps this repository's timed path; it is not available with --impl reference")
     if (args.roberta or args.kfac) and args.impl != "ours":
         print(json.dumps({"impl": args.impl, "unavailable": "--roberta / --kfac are measured for this repository only "
                           "(the reference arm runs the two headline configs)"}))
@@ -559,6 +589,7 @@ def main():
         for name, over in subs:
             sub = argparse.Namespace(**vars(args))
             sub.steps, sub.warmup, sub.no_e2e, sub.global_batch = min(args.steps, 4), 3, True, 0
+            sub.dump_outputs = None
             for k, v in over.items():
                 setattr(sub, k, v)
             gc.collect()
