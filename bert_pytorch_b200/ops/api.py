@@ -399,13 +399,6 @@ def attention_bwd(qkv, seqlens, ctx, dctx, lse, heads: int, *, p_drop=0.0, seed=
     return dqkv if fp8 is None else (dqkv, q)
 
 
-def set_attention_options(bwd_pipe: Optional[bool] = None, row_kernels: Optional[bool] = None) -> None:
-    """``bwd_pipe``: force the software-pipelined S > 128 backward kernel on / off; ``row_kernels``: force the
-    round-2 thread-per-query-row kernels on / off (None: follow B200_ATTN_BWD_PIPE / B200_ATTN_ROW, both default on)."""
-    extension().set_attention_options(-1 if bwd_pipe is None else int(bool(bwd_pipe)),
-                                      -1 if row_kernels is None else int(bool(row_kernels)))
-
-
 # ---------------------------------------------------------------------------
 # multi-tensor ops over arbitrary tensor lists
 # ---------------------------------------------------------------------------

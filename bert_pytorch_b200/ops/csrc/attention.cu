@@ -7,25 +7,22 @@
 // tiles of one head are plain 2-D TMA boxes of that matrix -- no permute/contiguous copies (K6 is gone);
 // the context is written as [B*S, H], ready for the output projection.
 //
-// Every kernel: 8 (or 16) math warps + 1 control warp.  The control warp's elected lane issues all TMA loads and
-// all tcgen05.mma; a query row (= TMEM lane) is shared by two (four) threads that own 64 (32) key columns each and
-// exchange row statistics through shared memory.
+// In every kernel elected lanes of control warps issue the TMA loads and the tcgen05.mma, and the math warps work on
+// rows of tensor memory (TMEM lane == query row).  Dropout draws Philox counter bits for the probabilities
+// (element ((b * h + head) * S + q) * S + k); the backward regenerates the same bits instead of storing a mask.
 //
-// Forward
-//   attn_fwd_single_kernel  S <= 128: one CTA per (batch, head); P overwrites the Q|K buffers, O overwrites the S
-//                           accumulator; 48 KB / 128 TMEM columns / 70 registers -> three CTAs per SM
-//   attn_fwd_kernel<2>      S > 128: one CTA per (batch, head, 128-query block); K blocks double buffered, one V
-//                           buffer, online softmax (fp32, exp2), O accumulated in registers from the TMEM result of
-//                           each key block; 96 KB / 256 columns -> two CTAs per SM
-//   dropout: Philox counter RNG on the probabilities, regenerated in the backward; P (bf16) goes to shared memory in
-//   the 128B-swizzled K-major layout the PV MMA reads.
-// Backward
-//   attn_bwd_single_kernel  S <= 128: one CTA per (batch, head); S = Q K^T, dP = dO V^T -> threads form P~, dS ->
-//                           dV = P~^T dO, dK = dS^T Q, dQ = dS K (transposes are free: MN-major descriptors on the
-//                           same tile); dV/dK/dQ overwrite the consumed S/dP accumulators, P~ and dS share one
-//                           buffer, delta = <dO, O> computed in-kernel; 96 KB / 256 columns -> two CTAs per SM
-//   attn_bwd_kernel         S > 128: one CTA per (batch, head, 128-key block) looping over the query blocks; dV, dK
-//                           accumulate in TMEM, dQ goes out per query block through fp32 atomics + a conversion pass
+// Forward: one thread per query row, P is written back into the S accumulator and feeds the P V MMA from TMEM
+//   attn_fwd_row_kernel     S <= 128: persistent CTAs over (batch, head); S, P and the P V result share 128 TMEM
+//                           columns, 48 KB -> four CTAs per SM
+//   attn_fwd_stream_kernel  S > 128: persistent CTAs over (batch, head, 128-query block); K / V two-stage ring, the
+//                           output accumulates in TMEM under a lazily raised running max; 256 columns -> two CTAs per SM
+// Backward: S = Q K^T, dP = dO V^T -> threads form P~ (dropped probabilities / keep_prob) and dS -> dV = P~^T dO,
+// dK = dS^T Q, dQ = dS K (the transposes are free: MN-major descriptors on the same tile)
+//   attn_bwd_row2_kernel    S <= 128: persistent CTAs over (batch, head), two threads per query row, delta = <dO, O>
+//                           in-kernel; dV / dK / dQ overwrite the consumed S / dP accumulators; 96 KB -> two CTAs per SM
+//   attn_bwd_pipe_kernel    S > 128: one CTA per (batch, head, 128-key block) looping over the query blocks, software
+//                           pipelined; dV, dK accumulate in TMEM, dQ goes out through fp32 atomics.  attn_delta_kernel
+//                           (delta = <dO, O>) runs before it, attn_dq_convert_kernel (fp32 dQ -> bf16) after it
 #include "common.cuh"
 #include "gemm_sm100.h"
 #include "kernels.h"
@@ -37,13 +34,7 @@ constexpr int ATT_BWD16_THREADS = 544; // streaming backward: 16 math warps (4 p
 constexpr int TILE = 128;          // query rows / key rows per block
 constexpr int HD = 64;             // head dim
 constexpr float LOG2E = 1.4426950408889634f;
-// -1: follow the environment (B200_ATTN_ROW, default on), 0 / 1: forced by attention_set_options
-static int g_attn_row = -1;
-static bool attn_row_enabled() {
-  if (g_attn_row >= 0) return g_attn_row != 0;
-  static const bool env_on = []() { const char* e = getenv("B200_ATTN_ROW"); return !(e && e[0] == '0'); }();
-  return env_on;
-}
+
 __device__ __forceinline__ float ex2_approx(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -88,405 +79,13 @@ __device__ __forceinline__ void emit_fp8_row(const Fp8Out& f8, size_t off, const
 }
 
 // ------------------------------------------------------------------------------------------------
-// forward
-// ------------------------------------------------------------------------------------------------
-// KV_STAGES = 1: the whole key range is one block (S <= 128): 80 KB of shared memory and 128 TMEM columns
-// (the PV result reuses the S columns) -> two CTAs per SM.  KV_STAGES = 2: K/V blocks stream through a ring.
-template <int KV_STAGES>
-__global__ void __launch_bounds__(ATT_BWD_THREADS, 2)
-attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const AttnArgs p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sQ = smem;                                  // 16 KB
-  uint8_t* sK = smem + 16384;                          // KV_STAGES x 16 KB
-  uint8_t* sV = sK + 16384 * KV_STAGES;                // 16 KB: ONE V buffer (it is needed late, after the softmax of
-                                                       // its block, so the next V streams in behind the PV MMA) -- keeps
-                                                       // the streaming variant at 96 KB: two CTAs per SM
-  uint8_t* sP = sV + 16384;                            // 32 KB
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sP + 32768);
-  constexpr uint32_t TMEM_COLS = KV_STAGES == 1 ? 128 : 256;
-  uint64_t* q_full = bars;               // 1
-  uint64_t* kv_full = bars + 1;          // 2
-  uint64_t* kv_empty = bars + 3;         // 2
-  uint64_t* s_ready = bars + 5;
-  uint64_t* p_ready = bars + 6;
-  uint64_t* pv_done = bars + 7;
-  uint64_t* v_full = bars + 8;
-  uint64_t* v_empty = bars + 9;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 10);
-  float* xch = reinterpret_cast<float*>(bars + 12);      // [2 buffers][2 halves][128 rows] row-max exchange (+ final sum)
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int qb = blockIdx.x, bh = blockIdx.y;
-  const int b = bh / p.h, head = bh % p.h;
-  const int seqlen = min(p.seqlens[b], p.S);
-  const int nkb = max(1, (seqlen + TILE - 1) / TILE);   // key blocks that contain valid keys
-  const int row0 = b * p.S;
-
-  if (threadIdx.x == 256) {
-    tma_prefetch_desc(&tmap_qkv);
-    mbar_init(q_full, 1);
-    for (int i = 0; i < 2; ++i) { mbar_init(&kv_full[i], 1); mbar_init(&kv_empty[i], 1); }
-    mbar_init(v_full, 1);
-    mbar_init(v_empty, 1);
-    mbar_init(s_ready, 1);
-    mbar_init(p_ready, 256);
-    mbar_init(pv_done, 1);
-    fence_barrier_init();
-  }
-  if (warp == 8) tmem_alloc(tmem_slot, TMEM_COLS);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const unsigned long long seed = p.thresh16 != 0 ? p.seed.value() : 0ull;
-  const uint32_t tS = tmem, tO = KV_STAGES == 1 ? tmem : tmem + 128;
-
-  if (warp == 8) {
-    if (lane == 0) {
-      const int cq = head * HD, ck = p.H + head * HD, cv = 2 * p.H + head * HD;
-      mbar_arrive_expect_tx(q_full, 16384);
-      tma_load_2d(sQ, &tmap_qkv, q_full, cq, row0 + qb * TILE);
-      // K blocks ride a KV_STAGES-deep ring (kv_full / kv_empty), V has one buffer (v_full / v_empty)
-      for (int j = 0; j < min(KV_STAGES, nkb); ++j) {
-        mbar_arrive_expect_tx(&kv_full[j], 16384);
-        tma_load_2d(sK + j * 16384, &tmap_qkv, &kv_full[j], ck, row0 + j * TILE);
-      }
-      mbar_arrive_expect_tx(v_full, 16384);
-      tma_load_2d(sV, &tmap_qkv, v_full, cv, row0);
-      constexpr uint32_t idesc_s = umma_idesc_bf16(128, 128, false, false);  // Q K^T : both K-major
-      constexpr uint32_t idesc_o = umma_idesc_bf16(128, 64, false, true);    // P V   : V is MN-major
-      mbar_wait(q_full, 0);
-      const uint64_t dq = umma_smem_desc_sw128(smem_u32(sQ), 16, 1024);
-      auto issue_s = [&](int j) {              // S_j = Q K_j^T, then the K slot is free for block j + KV_STAGES
-        const int st = KV_STAGES == 1 ? 0 : (j & 1);
-        mbar_wait(&kv_full[st], (j / KV_STAGES) & 1);
-        tc_fence_after();
-        const uint64_t dk = umma_smem_desc_sw128(smem_u32(sK + st * 16384), 16, 1024);
-#pragma unroll
-        for (int kk = 0; kk < HD / 16; ++kk) umma_bf16_ss(tS, dq + 2 * kk, dk + 2 * kk, idesc_s, kk > 0);
-        umma_commit(s_ready);
-        umma_commit(&kv_empty[st]);
-      };
-      issue_s(0);
-      for (int j = 0; j < nkb; ++j) {
-        const int st = KV_STAGES == 1 ? 0 : (j & 1);
-        if (j + KV_STAGES < nkb) {             // refill the K slot S_j just released
-          mbar_wait(&kv_empty[st], (j / KV_STAGES) & 1);
-          mbar_arrive_expect_tx(&kv_full[st], 16384);
-          tma_load_2d(sK + st * 16384, &tmap_qkv, &kv_full[st], ck, row0 + (j + KV_STAGES) * TILE);
-        }
-        mbar_wait(p_ready, j & 1);             // P_j is in shared memory (and S_j has been consumed)
-        mbar_wait(v_full, j & 1);
-        tc_fence_after();
-        const uint32_t ap = smem_u32(sP), av = smem_u32(sV);
-#pragma unroll
-        for (int kk = 0; kk < TILE / 16; ++kk) {
-          const uint64_t da = umma_smem_desc_sw128(ap + (kk >> 2) * 16384 + (kk & 3) * 32, 16, 1024);
-          const uint64_t db = umma_smem_desc_sw128(av + kk * 2048, 8192, 1024);
-          umma_bf16_ss(tO, da, db, idesc_o, kk > 0);
-        }
-        umma_commit(pv_done);
-        umma_commit(v_empty);
-        if (j + 1 < nkb) {
-          if (KV_STAGES > 1) issue_s(j + 1);   // the S accumulator is free: overlap Q K^T with the PV MMA's drain
-          mbar_wait(v_empty, j & 1);
-          mbar_arrive_expect_tx(v_full, 16384);
-          tma_load_2d(sV, &tmap_qkv, v_full, cv, row0 + (j + 1) * TILE);
-          if (KV_STAGES == 1) issue_s(j + 1);
-        }
-      }
-    }
-  } else {
-    // two threads per query row: thread (r, ch) owns key columns [64 ch, 64 ch + 64) of every key block and
-    // output columns [32 ch, 32 ch + 32); row maxima are exchanged through shared memory
-    const int r = (warp & 3) * 32 + lane;      // query row inside the tile == TMEM lane
-    const int ch = warp >> 2;
-    const int q = qb * TILE + r;               // query position in the sequence
-    const uint32_t lane_base = uint32_t((warp & 3) * 32) << 16;
-    const float c_scale = p.scale * LOG2E;
-    float m = -INFINITY, l = 0.f;
-    float o[32];
-#pragma unroll
-    for (int t = 0; t < 32; ++t) o[t] = 0.f;
-    const uint64_t erow = ((uint64_t)bh * p.S + (uint64_t)q) * (uint64_t)p.S;   // dropout element index base
-    for (int j = 0; j < nkb; ++j) {
-      mbar_wait(s_ready, j & 1);
-      tc_fence_after();
-      // pass 1: row max over the valid keys of this half block
-      float mx = -INFINITY;
-      const bool full = (j + 1) * TILE <= seqlen;         // every key of this block is valid (CTA uniform)
-#pragma unroll 1
-      for (int c = ch * 4; c < ch * 4 + 4; ++c) {        // 16-column sub-chunks keep the register count low
-        uint32_t v[16];
-        tmem_ld_32x16(tS + lane_base + c * 16, v);
-        tmem_ld_wait();
-        const int k0 = j * TILE + c * 16;
-        if (full) {
-#pragma unroll
-          for (int t = 0; t < 16; ++t) mx = fmaxf(mx, __uint_as_float(v[t]));
-        } else {
-#pragma unroll
-          for (int t = 0; t < 16; ++t)
-            if (k0 + t < seqlen) mx = fmaxf(mx, __uint_as_float(v[t]));
-        }
-      }
-      mx *= c_scale;                                      // c_scale > 0: max commutes with the scaling
-      float* xb = xch + (j & 1) * 256;
-      xb[ch * 128 + r] = mx;
-      asm volatile("bar.sync 1, 256;" ::: "memory");
-      mx = fmaxf(xb[r], xb[128 + r]);
-      const float m_new = fmaxf(m, mx);
-      const float alpha = (m == -INFINITY) ? 0.f : exp2f(m - m_new);
-      float rowsum = 0.f;
-      // pass 2: probabilities, dropout, P -> shared memory
-#pragma unroll 1
-      for (int c = ch * 4; c < ch * 4 + 4; ++c) {
-        uint32_t v[16];
-        tmem_ld_32x16(tS + lane_base + c * 16, v);
-        tmem_ld_wait();
-        const int k0 = j * TILE + c * 16;
-#pragma unroll
-        for (int g = 0; g < 2; ++g) {
-          float pr[8];
-#pragma unroll
-          for (int t = 0; t < 8; ++t) {
-            const int key = k0 + g * 8 + t;
-            float e = ex2_approx(fmaf(__uint_as_float(v[g * 8 + t]), c_scale, -m_new));
-            if (!full && key >= seqlen) e = 0.f;
-            rowsum += e;
-            pr[t] = e;
-          }
-          if (p.thresh16 != 0) {
-            const Keep8 keep = dropout_keep8(seed, p.stream, (erow + (uint64_t)(k0 + g * 8)) >> 3, p.thresh16);
-#pragma unroll
-            for (int t = 0; t < 8; ++t) pr[t] = keep[t] ? pr[t] * p.inv_keep : 0.f;
-          }
-          const uint4 pk = make_uint4(pack_bf16(pr[0], pr[1]), pack_bf16(pr[2], pr[3]), pack_bf16(pr[4], pr[5]),
-                                      pack_bf16(pr[6], pr[7]));
-          *reinterpret_cast<uint4*>(sP + p_chunk_offset(r, c * 2 + g)) = pk;
-        }
-      }
-      l = l * alpha + rowsum;                  // this half's share of the denominator
-      m = m_new;
-#pragma unroll
-      for (int t = 0; t < 32; ++t) o[t] *= alpha;
-      fence_proxy_async();       // generic-proxy smem writes -> visible to the tensor core (async proxy)
-      tc_fence_before();
-      mbar_arrive(p_ready);
-      mbar_wait(pv_done, j & 1);
-      tc_fence_after();
-      {
-        uint32_t v[32];
-        tmem_ld_32x32(tO + lane_base + ch * 32, v);
-        tmem_ld_wait();
-#pragma unroll
-        for (int t = 0; t < 32; ++t) o[t] += __uint_as_float(v[t]);
-      }
-    }
-    float* xs = xch + 512;                     // final exchange of the two partial denominators
-    xs[ch * 128 + r] = l;
-    asm volatile("bar.sync 1, 256;" ::: "memory");
-    l = xs[r] + xs[128 + r];
-    if (q < p.S) {
-      const float inv_l = 1.f / l;
-      __nv_bfloat16* dst = p.ctx + (size_t)(row0 + q) * p.H + head * HD + ch * 32;
-#pragma unroll
-      for (int g = 0; g < 4; ++g)
-        *reinterpret_cast<uint4*>(dst + g * 8) =
-            make_uint4(pack_bf16(o[g * 8] * inv_l, o[g * 8 + 1] * inv_l), pack_bf16(o[g * 8 + 2] * inv_l, o[g * 8 + 3] * inv_l),
-                       pack_bf16(o[g * 8 + 4] * inv_l, o[g * 8 + 5] * inv_l), pack_bf16(o[g * 8 + 6] * inv_l, o[g * 8 + 7] * inv_l));
-      if (p.f8.q) {
-        float amax = 0.f;
-        const float qscale = p.f8.meta[1];
-#pragma unroll
-        for (int g = 0; g < 4; ++g) {
-          float t8[8];
-#pragma unroll
-          for (int t = 0; t < 8; ++t) t8[t] = o[g * 8 + t] * inv_l;
-          fp8_emit8(p.f8, (size_t)(row0 + q) * p.H + head * HD + ch * 32 + g * 8, t8, qscale, amax);
-        }
-        if (amax > 0.f) atomicMax(reinterpret_cast<int*>(p.f8.meta), __float_as_int(isfinite(amax) ? amax : 3.0e38f));
-      }
-      if (ch == 0) p.lse[(size_t)bh * p.S + q] = (m + log2f(l)) * 0.6931471805599453f;
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 8) {
-    tc_fence_after();
-    tmem_dealloc(tmem, TMEM_COLS);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// forward, S <= 128 (phase 1): one query block and one key block per (batch, head).  No online-softmax state, the
-// probabilities overwrite the Q|K operand buffers once S = Q K^T has retired (48 KB of shared memory), the PV
-// result overwrites the S columns (128 TMEM columns) and the softmax needs < 75 registers: three CTAs per SM
-// instead of two, which is what this latency-bound kernel (one dependent chain per head) is short of.
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(ATT_BWD_THREADS, 3)
-attn_fwd_single_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const AttnArgs p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sQ = smem;                                  // 16 KB  } P (32 KB) lands here after the S MMA
-  uint8_t* sK = smem + 16384;                          // 16 KB  }
-  uint8_t* sV = smem + 32768;                          // 16 KB
-  uint8_t* sP = smem;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 49152);
-  uint64_t* in_full = bars;
-  uint64_t* s_ready = bars + 1;
-  uint64_t* p_ready = bars + 2;
-  uint64_t* pv_done = bars + 3;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4);
-  float* xch = reinterpret_cast<float*>(bars + 6);     // [2 exchanges][2 halves][128 rows]
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int bh = blockIdx.y;
-  const int b = bh / p.h, head = bh % p.h;
-  const int seqlen = min(p.seqlens[b], p.S);
-  const int row0 = b * p.S;
-
-  if (threadIdx.x == 256) {
-    tma_prefetch_desc(&tmap_qkv);
-    mbar_init(in_full, 1);
-    mbar_init(s_ready, 1);
-    mbar_init(p_ready, 256);
-    mbar_init(pv_done, 1);
-    fence_barrier_init();
-  }
-  if (warp == 8) tmem_alloc(tmem_slot, 128);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tS = *tmem_slot;
-  const unsigned long long seed = p.thresh16 != 0 ? p.seed.value() : 0ull;
-
-  if (warp == 8) {
-    if (lane == 0) {
-      mbar_arrive_expect_tx(in_full, 49152);
-      tma_load_2d(sQ, &tmap_qkv, in_full, head * HD, row0);
-      tma_load_2d(sK, &tmap_qkv, in_full, p.H + head * HD, row0);
-      tma_load_2d(sV, &tmap_qkv, in_full, 2 * p.H + head * HD, row0);
-      constexpr uint32_t idesc_s = umma_idesc_bf16(128, 128, false, false);  // Q K^T : both K-major
-      constexpr uint32_t idesc_o = umma_idesc_bf16(128, 64, false, true);    // P V   : V is MN-major
-      mbar_wait(in_full, 0);
-      tc_fence_after();
-      const uint64_t dq = umma_smem_desc_sw128(smem_u32(sQ), 16, 1024);
-      const uint64_t dk = umma_smem_desc_sw128(smem_u32(sK), 16, 1024);
-#pragma unroll
-      for (int kk = 0; kk < HD / 16; ++kk) umma_bf16_ss(tS, dq + 2 * kk, dk + 2 * kk, idesc_s, kk > 0);
-      umma_commit(s_ready);                    // also: Q and K are no longer read -> P may overwrite them
-      mbar_wait(p_ready, 0);
-      tc_fence_after();
-      const uint32_t ap = smem_u32(sP), av = smem_u32(sV);
-#pragma unroll
-      for (int kk = 0; kk < TILE / 16; ++kk) {
-        const uint64_t da = umma_smem_desc_sw128(ap + (kk >> 2) * 16384 + (kk & 3) * 32, 16, 1024);
-        const uint64_t db = umma_smem_desc_sw128(av + kk * 2048, 8192, 1024);
-        umma_bf16_ss(tS, da, db, idesc_o, kk > 0);   // O -> columns [0, 64) of the (consumed) S accumulator
-      }
-      umma_commit(pv_done);
-    }
-  } else {
-    // two threads per query row: thread (r, ch) owns key columns [64 ch, 64 ch + 64) and output columns [32 ch, 32 ch + 32)
-    const int r = (warp & 3) * 32 + lane;
-    const int ch = warp >> 2;
-    const uint32_t lane_base = uint32_t((warp & 3) * 32) << 16;
-    const float c_scale = p.scale * LOG2E;
-    const uint64_t erow = ((uint64_t)bh * p.S + (uint64_t)r) * (uint64_t)p.S;
-    const bool full = TILE <= seqlen;
-    mbar_wait(s_ready, 0);
-    tc_fence_after();
-    float mx = -INFINITY;
-#pragma unroll 1
-    for (int c = ch * 4; c < ch * 4 + 4; ++c) {
-      uint32_t v[16];
-      tmem_ld_32x16(tS + lane_base + c * 16, v);
-      tmem_ld_wait();
-      if (full) {
-#pragma unroll
-        for (int t = 0; t < 16; ++t) mx = fmaxf(mx, __uint_as_float(v[t]));
-      } else {
-#pragma unroll
-        for (int t = 0; t < 16; ++t)
-          if (c * 16 + t < seqlen) mx = fmaxf(mx, __uint_as_float(v[t]));
-      }
-    }
-    mx *= c_scale;
-    xch[ch * 128 + r] = mx;
-    asm volatile("bar.sync 1, 256;" ::: "memory");
-    const float m = fmaxf(fmaxf(xch[r], xch[128 + r]), -1e30f);   // an all-padding row stays finite
-    float rowsum = 0.f;
-#pragma unroll 1
-    for (int c = ch * 4; c < ch * 4 + 4; ++c) {
-      uint32_t v[16];
-      tmem_ld_32x16(tS + lane_base + c * 16, v);
-      tmem_ld_wait();
-#pragma unroll
-      for (int g = 0; g < 2; ++g) {
-        float pr[8];
-#pragma unroll
-        for (int t = 0; t < 8; ++t) {
-          float e = ex2_approx(fmaf(__uint_as_float(v[g * 8 + t]), c_scale, -m));
-          if (!full && c * 16 + g * 8 + t >= seqlen) e = 0.f;
-          rowsum += e;
-          pr[t] = e;
-        }
-        if (p.thresh16 != 0) {
-          const Keep8 keep = dropout_keep8(seed, p.stream, (erow + (uint64_t)(c * 16 + g * 8)) >> 3, p.thresh16);
-#pragma unroll
-          for (int t = 0; t < 8; ++t) pr[t] = keep[t] ? pr[t] * p.inv_keep : 0.f;
-        }
-        *reinterpret_cast<uint4*>(sP + p_chunk_offset(r, c * 2 + g)) =
-            make_uint4(pack_bf16(pr[0], pr[1]), pack_bf16(pr[2], pr[3]), pack_bf16(pr[4], pr[5]), pack_bf16(pr[6], pr[7]));
-      }
-    }
-    xch[256 + ch * 128 + r] = rowsum;
-    fence_proxy_async();       // generic-proxy smem writes -> visible to the tensor core (async proxy)
-    tc_fence_before();         // S reads retired before the PV MMA overwrites those columns
-    mbar_arrive(p_ready);
-    asm volatile("bar.sync 1, 256;" ::: "memory");
-    const float l = xch[256 + r] + xch[256 + 128 + r];
-    mbar_wait(pv_done, 0);
-    tc_fence_after();
-    uint32_t o[32];
-    tmem_ld_32x32(tS + lane_base + ch * 32, o);
-    tmem_ld_wait();
-    if (r < p.S) {
-      const float inv_l = 1.f / l;
-      __nv_bfloat16* dst = p.ctx + (size_t)(row0 + r) * p.H + head * HD + ch * 32;
-#pragma unroll
-      for (int g = 0; g < 4; ++g)
-        *reinterpret_cast<uint4*>(dst + g * 8) = make_uint4(
-            pack_bf16(__uint_as_float(o[g * 8]) * inv_l, __uint_as_float(o[g * 8 + 1]) * inv_l),
-            pack_bf16(__uint_as_float(o[g * 8 + 2]) * inv_l, __uint_as_float(o[g * 8 + 3]) * inv_l),
-            pack_bf16(__uint_as_float(o[g * 8 + 4]) * inv_l, __uint_as_float(o[g * 8 + 5]) * inv_l),
-            pack_bf16(__uint_as_float(o[g * 8 + 6]) * inv_l, __uint_as_float(o[g * 8 + 7]) * inv_l));
-      if (p.f8.q) {
-        float amax = 0.f;
-        emit_fp8_row<4>(p.f8, (size_t)(row0 + r) * p.H + head * HD + ch * 32, o, inv_l, p.f8.meta[1], amax);
-        if (amax > 0.f) atomicMax(reinterpret_cast<int*>(p.f8.meta), __float_as_int(isfinite(amax) ? amax : 3.0e38f));
-      }
-      if (ch == 0) p.lse[(size_t)bh * p.S + r] = (m + log2f(l)) * 0.6931471805599453f;
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 8) {
-    tc_fence_after();
-    tmem_dealloc(tS, 128);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Round-2 forward: one THREAD per query row, P stays in tensor memory, persistent CTAs.
+// forward: one THREAD per query row, P stays in tensor memory, persistent CTAs.
 //
-// ncu on the kernels above (profiles/ncu_hot_kernels_r1.md): 23-25 instructions per score element at ~55 % issue
-// utilisation and 8-10 % tensor-pipe activity -- the softmax, not the MMA, is the cost, and half of it is overhead
-// of the two-threads-per-row mapping (two TMEM passes of 16-column loads, shared-memory exchanges and block
-// barriers for the row statistics, swizzled shared-memory stores of P, Philox key schedule and 16-bit field
-// extraction per element).  Here
+// The softmax, not the MMA, is the cost of the forward: a two-threads-per-row layout measured 23-25 instructions per
+// score element at ~55 % issue utilisation and 8-10 % tensor-pipe activity (profiles/ncu_hot_kernels_r1.md), half of
+// it overhead of that mapping (two TMEM passes of 16-column loads, shared-memory exchanges and block barriers for the
+// row statistics, swizzled shared-memory stores of P, Philox key schedule and 16-bit field extraction per element).
+// Here
 //   * thread r of the four softmax warps owns TMEM lane r = query row r: row max / row sum never leave the thread
 //     (no exchange, no barrier), 3-input max, 32-column TMEM loads with the next chunk in flight;
 //   * P (bf16) is written back into the first 64 columns of the S accumulator with tcgen05.st and feeds the PV MMA
@@ -961,265 +560,22 @@ attn_delta_kernel(const __nv_bfloat16* __restrict__ o, const __nv_bfloat16* __re
   }
 }
 
-// 16 math warps: four threads per query row (TMEM lane quarter = warp & 3, 32-key column quarter = warp >> 2).  With
-// one CTA per SM (512 TMEM columns, 160 KB) the kernel is bound by the latency of the per-thread softmax-gradient
-// chain; twice the warps halve it.  16-column TMEM loads keep the kernel under the 120 registers 544 threads allow.
-__global__ void __launch_bounds__(ATT_BWD16_THREADS, 1)
-attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_do,
-                const AttnArgs p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sK = smem;                      // 16 KB
-  uint8_t* sV = smem + 16384;              // 16 KB
-  uint8_t* sQ = smem + 16384 * 2;          // 2 x 16 KB
-  uint8_t* sDO = smem + 16384 * 4;         // 2 x 16 KB
-  uint8_t* sPd = smem + 16384 * 6;         // 32 KB
-  uint8_t* sDS = smem + 16384 * 8;         // 32 KB
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 16384 * 10);
-  uint64_t* kv_full = bars;
-  uint64_t* qdo_full = bars + 1;           // 2
-  uint64_t* qdo_empty = bars + 3;          // 2
-  uint64_t* sdp_ready = bars + 5;
-  uint64_t* ds_ready = bars + 6;
-  uint64_t* dq_ready = bars + 7;
-  uint64_t* fin = bars + 8;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 9);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int kb = blockIdx.x, bh = blockIdx.y;
-  const int b = bh / p.h, head = bh % p.h;
-  const int seqlen = min(p.seqlens[b], p.S);
-  const int nqb = (p.S + TILE - 1) / TILE;
-  const int nkb_total = gridDim.x;
-  const int row0 = b * p.S;
-  const bool dead = kb * TILE >= seqlen;     // every key of this block is padding: dK = dV = 0
-
-  if (dead) {
-    if (warp < 4) {
-      const int key = kb * TILE + warp * 32 + lane;
-      if (key < p.S) {
-        __nv_bfloat16* dk = p.dqkv + (size_t)(row0 + key) * 3 * p.H + p.H + head * HD;
-        __nv_bfloat16* dv = dk + p.H;
-#pragma unroll
-        for (int g = 0; g < 8; ++g) {
-          *reinterpret_cast<uint4*>(dk + g * 8) = make_uint4(0, 0, 0, 0);
-          *reinterpret_cast<uint4*>(dv + g * 8) = make_uint4(0, 0, 0, 0);
-        }
-        if (p.f8.q) {
-          unsigned char* qk = p.f8.q + (size_t)(row0 + key) * 3 * p.H + p.H + head * HD;
-#pragma unroll
-          for (int g = 0; g < 4; ++g) {
-            *reinterpret_cast<uint4*>(qk + g * 16) = make_uint4(0, 0, 0, 0);
-            *reinterpret_cast<uint4*>(qk + p.H + g * 16) = make_uint4(0, 0, 0, 0);
-          }
-        }
-      }
-    }
-    return;
-  }
-
-  if (threadIdx.x == 512) {
-    tma_prefetch_desc(&tmap_qkv);
-    tma_prefetch_desc(&tmap_do);
-    mbar_init(kv_full, 1);
-    for (int i = 0; i < 2; ++i) { mbar_init(&qdo_full[i], 1); mbar_init(&qdo_empty[i], 1); }
-    mbar_init(sdp_ready, 1);
-    mbar_init(ds_ready, 512);
-    mbar_init(dq_ready, 1);
-    mbar_init(fin, 1);
-    fence_barrier_init();
-  }
-  if (warp == 16) tmem_alloc(tmem_slot, 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const unsigned long long seed = p.thresh16 != 0 ? p.seed.value() : 0ull;
-  const uint32_t tS = tmem, tDP = tmem + 128, tDV = tmem + 256, tDK = tmem + 320, tDQ = tmem + 384;
-
-  if (warp == 16) {
-    if (lane == 0) {
-      const int cq = head * HD, ck = p.H + head * HD, cv = 2 * p.H + head * HD;
-      mbar_arrive_expect_tx(kv_full, 32768);
-      tma_load_2d(sK, &tmap_qkv, kv_full, ck, row0 + kb * TILE);
-      tma_load_2d(sV, &tmap_qkv, kv_full, cv, row0 + kb * TILE);
-      for (int i = 0; i < min(2, nqb); ++i) {
-        mbar_arrive_expect_tx(&qdo_full[i], 32768);
-        tma_load_2d(sQ + i * 16384, &tmap_qkv, &qdo_full[i], cq, row0 + i * TILE);
-        tma_load_2d(sDO + i * 16384, &tmap_do, &qdo_full[i], head * HD, row0 + i * TILE);
-      }
-      constexpr uint32_t id_kk = umma_idesc_bf16(128, 128, false, false);  // [q x keys], both K-major
-      constexpr uint32_t id_tt = umma_idesc_bf16(128, 64, true, true);     // [keys x d] = X^T Y, both MN-major
-      constexpr uint32_t id_kt = umma_idesc_bf16(128, 64, false, true);    // [q x d] = dS K, A K-major, B MN-major
-      mbar_wait(kv_full, 0);
-      for (int i = 0; i < nqb; ++i) {
-        const int st = i & 1;
-        mbar_wait(&qdo_full[st], (i >> 1) & 1);
-        tc_fence_after();
-        const uint32_t aq = smem_u32(sQ + st * 16384), ado = smem_u32(sDO + st * 16384);
-        const uint32_t ak = smem_u32(sK), av = smem_u32(sV), apd = smem_u32(sPd), ads = smem_u32(sDS);
-#pragma unroll
-        for (int kk = 0; kk < HD / 16; ++kk)   // S = Q K^T
-          umma_bf16_ss(tS, umma_smem_desc_sw128(aq + kk * 32, 16, 1024), umma_smem_desc_sw128(ak + kk * 32, 16, 1024),
-                       id_kk, kk > 0);
-#pragma unroll
-        for (int kk = 0; kk < HD / 16; ++kk)   // dPd = dO V^T
-          umma_bf16_ss(tDP, umma_smem_desc_sw128(ado + kk * 32, 16, 1024), umma_smem_desc_sw128(av + kk * 32, 16, 1024),
-                       id_kk, kk > 0);
-        umma_commit(sdp_ready);
-        mbar_wait(ds_ready, i & 1);
-        tc_fence_after();
-#pragma unroll
-        for (int kk = 0; kk < TILE / 16; ++kk) {   // reduction over the 128 query rows of this block
-          // A^T tiles: [q rows][keys] read MN-major (M = keys: two 64-wide blocks 16 KB apart)
-          const uint64_t a_pd = umma_smem_desc_sw128(apd + kk * 2048, 16384, 1024);
-          const uint64_t a_ds = umma_smem_desc_sw128(ads + kk * 2048, 16384, 1024);
-          const uint64_t b_do = umma_smem_desc_sw128(ado + kk * 2048, 8192, 1024);
-          const uint64_t b_q = umma_smem_desc_sw128(aq + kk * 2048, 8192, 1024);
-          umma_bf16_ss(tDV, a_pd, b_do, id_tt, (i > 0 || kk > 0));   // dV += Pd^T dO
-          umma_bf16_ss(tDK, a_ds, b_q, id_tt, (i > 0 || kk > 0));    // dK += dS^T Q
-        }
-#pragma unroll
-        for (int kk = 0; kk < TILE / 16; ++kk) {   // dQ = dS K   (reduction over the 128 keys)
-          const uint64_t a_ds = umma_smem_desc_sw128(ads + (kk >> 2) * 16384 + (kk & 3) * 32, 16, 1024);
-          const uint64_t b_k = umma_smem_desc_sw128(ak + kk * 2048, 8192, 1024);
-          umma_bf16_ss(tDQ, a_ds, b_k, id_kt, kk > 0);
-        }
-        umma_commit(dq_ready);
-        umma_commit(&qdo_empty[st]);
-        if (i + 2 < nqb) {
-          mbar_wait(&qdo_empty[st], (i >> 1) & 1);
-          mbar_arrive_expect_tx(&qdo_full[st], 32768);
-          tma_load_2d(sQ + st * 16384, &tmap_qkv, &qdo_full[st], cq, row0 + (i + 2) * TILE);
-          tma_load_2d(sDO + st * 16384, &tmap_do, &qdo_full[st], head * HD, row0 + (i + 2) * TILE);
-        }
-      }
-      umma_commit(fin);
-    }
-  } else {
-    const int r = (warp & 3) * 32 + lane;        // query row inside the tile == TMEM lane
-    const int ch = warp >> 2;                    // which 32-key column quarter this thread handles
-    const uint32_t lane_base = uint32_t((warp & 3) * 32) << 16;
-    const float c_scale = p.scale * LOG2E;
-    const float qscale8 = p.f8.q ? p.f8.meta[1] : 0.f;
-    float amax8 = 0.f;
-    for (int i = 0; i < nqb; ++i) {
-      const int q = i * TILE + r;
-      const bool q_ok = q < p.S;
-      const float lse2 = q_ok ? p.lse[(size_t)bh * p.S + q] * LOG2E : 0.f;
-      const float dlt = q_ok ? p.delta[(size_t)bh * p.S + q] : 0.f;
-      const uint64_t erow = ((uint64_t)bh * p.S + (uint64_t)q) * (uint64_t)p.S;
-      mbar_wait(sdp_ready, i & 1);
-      tc_fence_after();
-#pragma unroll
-      for (int sc = 0; sc < 2; ++sc) {           // two 16-column sub-chunks
-        const int c16 = ch * 2 + sc;
-        uint32_t sv[16], dv[16];
-        tmem_ld_32x16(tS + lane_base + c16 * 16, sv);
-        tmem_ld_32x16(tDP + lane_base + c16 * 16, dv);
-        tmem_ld_wait();
-        const int k0 = kb * TILE + c16 * 16;
-#pragma unroll
-        for (int g = 0; g < 2; ++g) {
-          Keep8 keep = Keep8::all();
-          if (p.thresh16 != 0)
-            keep = dropout_keep8(seed, p.stream, (erow + (uint64_t)(k0 + g * 8)) >> 3, p.thresh16);
-          float pd[8], ds[8];
-#pragma unroll
-          for (int t = 0; t < 8; ++t) {
-            const int key = k0 + g * 8 + t;
-            const bool ok = q_ok && key < seqlen;
-            const float pr = ok ? ex2_approx(fmaf(__uint_as_float(sv[g * 8 + t]), c_scale, -lse2)) : 0.f;
-            const bool kp = keep[t];
-            const float dp = kp ? __uint_as_float(dv[g * 8 + t]) * p.inv_keep : 0.f;
-            pd[t] = kp ? pr * p.inv_keep : 0.f;
-            ds[t] = pr * (dp - dlt) * p.scale;
-          }
-          const uint32_t off = p_chunk_offset(r, c16 * 2 + g);
-          *reinterpret_cast<uint4*>(sPd + off) = make_uint4(pack_bf16(pd[0], pd[1]), pack_bf16(pd[2], pd[3]),
-                                                            pack_bf16(pd[4], pd[5]), pack_bf16(pd[6], pd[7]));
-          *reinterpret_cast<uint4*>(sDS + off) = make_uint4(pack_bf16(ds[0], ds[1]), pack_bf16(ds[2], ds[3]),
-                                                            pack_bf16(ds[4], ds[5]), pack_bf16(ds[6], ds[7]));
-        }
-      }
-      fence_proxy_async();
-      tc_fence_before();
-      mbar_arrive(ds_ready);
-      mbar_wait(dq_ready, i & 1);
-      tc_fence_after();
-      {
-        uint32_t v[16];                          // each thread writes 16 of the 64 dQ columns of its row
-        tmem_ld_32x16(tDQ + lane_base + ch * 16, v);
-        tmem_ld_wait();
-        if (q_ok) {
-          if (nkb_total == 1) {
-            __nv_bfloat16* dq = p.dqkv + (size_t)(row0 + q) * 3 * p.H + head * HD + ch * 16;
-#pragma unroll
-            for (int g = 0; g < 2; ++g)
-              *reinterpret_cast<uint4*>(dq + g * 8) = make_uint4(
-                  pack_bf16(__uint_as_float(v[g * 8]), __uint_as_float(v[g * 8 + 1])),
-                  pack_bf16(__uint_as_float(v[g * 8 + 2]), __uint_as_float(v[g * 8 + 3])),
-                  pack_bf16(__uint_as_float(v[g * 8 + 4]), __uint_as_float(v[g * 8 + 5])),
-                  pack_bf16(__uint_as_float(v[g * 8 + 6]), __uint_as_float(v[g * 8 + 7])));
-            if (p.f8.q) emit_fp8_row<2>(p.f8, (size_t)(row0 + q) * 3 * p.H + head * HD + ch * 16, v, 1.f, qscale8, amax8);
-          } else {
-            float* dq = p.dq_acc + (size_t)(row0 + q) * p.H + head * HD + ch * 16;
-#pragma unroll
-            for (int g = 0; g < 4; ++g)
-              asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dq + g * 4),
-                           "f"(__uint_as_float(v[g * 4])), "f"(__uint_as_float(v[g * 4 + 1])),
-                           "f"(__uint_as_float(v[g * 4 + 2])), "f"(__uint_as_float(v[g * 4 + 3]))
-                           : "memory");
-          }
-        }
-      }
-      tc_fence_before();   // dQ TMEM reads done before the next block's MMA may overwrite it
-    }
-    // dK / dV of this key block: column quarters 0,1 write the two halves of dK, quarters 2,3 those of dV
-    mbar_wait(fin, 0);
-    tc_fence_after();
-    const int key = kb * TILE + r;
-    {
-      const int w = ch >> 1, c = ch & 1;
-      const uint32_t src = w == 0 ? tDK : tDV;
-      uint32_t v[32];
-      tmem_ld_32x32(src + lane_base + c * 32, v);
-      tmem_ld_wait();
-      if (key < p.S) {
-        __nv_bfloat16* dst = p.dqkv + (size_t)(row0 + key) * 3 * p.H + (w + 1) * p.H + head * HD + c * 32;
-#pragma unroll
-        for (int g = 0; g < 4; ++g)
-          *reinterpret_cast<uint4*>(dst + g * 8) = make_uint4(
-              pack_bf16(__uint_as_float(v[g * 8]), __uint_as_float(v[g * 8 + 1])),
-              pack_bf16(__uint_as_float(v[g * 8 + 2]), __uint_as_float(v[g * 8 + 3])),
-              pack_bf16(__uint_as_float(v[g * 8 + 4]), __uint_as_float(v[g * 8 + 5])),
-              pack_bf16(__uint_as_float(v[g * 8 + 6]), __uint_as_float(v[g * 8 + 7])));
-        if (p.f8.q)
-          emit_fp8_row<4>(p.f8, (size_t)(row0 + key) * 3 * p.H + (w + 1) * p.H + head * HD + c * 32, v, 1.f, qscale8, amax8);
-      }
-    }
-    if (p.f8.q) fp8_amax_commit(p.f8, amax8);
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 16) {
-    tc_fence_after();
-    tmem_dealloc(tmem, 512);
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
-// backward, S > 128, software-pipelined variant (opt-in: B200_ATTN_BWD_PIPE=1 / set_attention_options).
-// The kernel above runs its per-query-block stages strictly one after the other (S/dP MMAs -> softmax-gradient
-// math -> dV/dK/dQ MMAs -> dQ reduction): ~6 us per block of which < 1 us is tensor work.  Here
+// backward, S > 128: one CTA per (batch, head, 128-key block), looping over the query blocks.  16 math warps: four
+// threads per query row (TMEM lane quarter = warp & 3, 32-key column quarter = warp >> 2) -- at one CTA per SM the
+// latency of the per-thread softmax-gradient chain bounds the kernel, and more threads per row shorten it; 16-column
+// TMEM loads keep it under the 120 registers 544 threads allow.  TMEM (512 columns): S | dP | dV | dK | dQ.  Per query
+// block the math warps write P~ and dS to shared memory (32 KB each, in the 128B-swizzled layout the MMAs read); dV +=
+// P~^T dO and dK += dS^T Q accumulate in TMEM over all query blocks, dQ = dS K of the block is added to the fp32 dQ
+// accumulator with vector atomics.  A key block that is all padding writes zero dK / dV and exits.  Pipelining:
 //   * the math warps release S/dP as soon as they have pulled them out of TMEM (`sdp_free`), so the S/dP MMAs of
 //     block i+1 run while block i's math is still in registers;
 //   * block i's dQ is read back one iteration later (after block i+1's S/dP were loaded), so the dV/dK/dQ MMAs of
 //     block i overlap the math of block i+1;
 //   * Q/dO live in a 3-stage ring (blocks i, i+1 in use, i+2 landing); the reload of a stage is issued one iteration
 //     after its last reader, when the wait is free.
-// TMEM / P~ / dS buffers are unchanged (the hazards are covered by dq_ready(i-1) -> stores of block i, and
-// ds_ready(i) -> dQ MMA of block i).  192 KB shared memory, one CTA per SM.
+// One P~ and one dS buffer serve every block: dq_ready(i-1) orders the stores of block i after the MMAs that read
+// block i-1's, and ds_ready(i) orders the dQ MMA of block i after those stores.  192 KB shared memory, one CTA per SM.
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(ATT_BWD16_THREADS, 1)
 attn_bwd_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_do,
@@ -1489,239 +845,25 @@ attn_bwd_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_
 }
 
 // ------------------------------------------------------------------------------------------------
-// backward, S <= 128 (phase 1): ONE key block and ONE query block per (batch, head), so nothing accumulates across
-// iterations and the kernel can be made small enough for TWO CTAs per SM (the generic kernel is latency bound at
-// one CTA per SM: ~11 us per head, almost all of it dependent waits):
-//   * TMEM 256 columns: S | dP; dV then overwrites S[0,64), dK S[64,128) and dQ dP[0,64) -- by then every thread
-//     has consumed S and dP
-//   * ONE 32 KB operand buffer for P~ (dropped probabilities) and dS: P~ goes out first and feeds dV = P~^T dO while
-//     the threads keep dS packed in 32 registers; once that MMA has retired the same buffer receives dS for
-//     dK = dS^T Q and dQ = dS K
-//   * 96 KB of shared memory, <= 112 registers
+// backward, S <= 128: TWO threads per query row (64 key columns each, 8 math warps), persistent CTAs over
+// (batch, head) items, dS PARKED IN TENSOR MEMORY.  The MMA chain: S = Q K^T, dP = dO V^T -> P~ -> dV = P~^T dO;
+// dS -> dK = dS^T Q, dQ = dS K; dV / dK / dQ overwrite the consumed S / dP accumulators, one 32 KB buffer carries P~
+// and then dS.  A one-thread-per-row layout of the same chain measured 19 % issue utilisation (NOTES.md): four math
+// warps per CTA cannot hide the dependent MMA -> math -> MMA -> math -> MMA chain and the global loads of O / lse at
+// the head of an item, and its 64 registers of packed dS forced full unrolling (instruction-cache misses).  Here
+//   * ~12 instructions per score element (dsoftmax_chunk16): 1 / keep_prob in the exponent, dS = p' * select(keep,
+//     dP * scale + c, c) with the row constants folded, hoisted Philox keys, in-place 16-bit keep compares;
+//   * every 16-column chunk's dS (8 packed words) is written back with tcgen05.st into the upper half of the thread's
+//     own, already consumed dP columns (chunks run right to left, so the target columns are always behind the read
+//     pointer) and copied to shared memory once the dV MMA has released the P~ buffer: no register array survives the
+//     chunk loop, which therefore stays rolled (small code, 16-byte shared-memory stores);
+//   * the loop over items keeps TMEM / barriers alive, V of the next item streams in under the softmax-gradient math
+//     and Q / K / dO under the epilogue stores; the O half-row and log-sum-exp of the NEXT item are fetched while this
+//     item waits for its last MMAs;
+//   * delta = <dO, O>: each thread of a row computes half, one shared-memory exchange + named barrier per item.
+// 96 KB, 256 TMEM columns, 288 threads -> two CTAs per SM (16 math warps per SM).
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(ATT_BWD_THREADS, 2)
-attn_bwd_single_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_do,
-                       const AttnArgs p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sK = smem;                      // 16 KB each
-  uint8_t* sV = smem + 16384;
-  uint8_t* sQ = smem + 16384 * 2;
-  uint8_t* sDO = smem + 16384 * 3;
-  uint8_t* sP = smem + 16384 * 4;          // 32 KB: P~, later dS
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 16384 * 6);
-  uint64_t* in_full = bars;                // Q, K, V, dO landed
-  uint64_t* sdp_ready = bars + 1;          // S and dP accumulators complete
-  uint64_t* pd_ready = bars + 2;           // 256 threads: P~ is in shared memory
-  uint64_t* dv_done = bars + 3;            // dV MMA retired: the buffer may be overwritten with dS
-  uint64_t* ds_ready = bars + 4;           // 256 threads: dS is in shared memory
-  uint64_t* fin = bars + 5;                // dK, dQ complete
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 6);
-  float* xch = reinterpret_cast<float*>(bars + 8);   // [2 halves][128 rows]: partial delta = <dO, O> of a row
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int bh = blockIdx.y;
-  const int b = bh / p.h, head = bh % p.h;
-  const int seqlen = min(p.seqlens[b], p.S);
-  const int row0 = b * p.S;
-
-  if (threadIdx.x == 256) {
-    tma_prefetch_desc(&tmap_qkv);
-    tma_prefetch_desc(&tmap_do);
-    mbar_init(in_full, 1);
-    mbar_init(sdp_ready, 1);
-    mbar_init(pd_ready, 256);
-    mbar_init(dv_done, 1);
-    mbar_init(ds_ready, 256);
-    mbar_init(fin, 1);
-    fence_barrier_init();
-  }
-  if (warp == 8) tmem_alloc(tmem_slot, 256);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const unsigned long long seed = p.thresh16 != 0 ? p.seed.value() : 0ull;
-  const uint32_t tS = tmem, tDP = tmem + 128, tDV = tmem, tDK = tmem + 64, tDQ = tmem + 128;
-
-  if (warp == 8) {
-    if (lane == 0) {
-      const int cq = head * HD, ck = p.H + head * HD, cv = 2 * p.H + head * HD;
-      mbar_arrive_expect_tx(in_full, 65536);
-      tma_load_2d(sK, &tmap_qkv, in_full, ck, row0);
-      tma_load_2d(sV, &tmap_qkv, in_full, cv, row0);
-      tma_load_2d(sQ, &tmap_qkv, in_full, cq, row0);
-      tma_load_2d(sDO, &tmap_do, in_full, head * HD, row0);
-      constexpr uint32_t id_kk = umma_idesc_bf16(128, 128, false, false);  // [q x keys], both K-major
-      constexpr uint32_t id_tt = umma_idesc_bf16(128, 64, true, true);     // [keys x d] = X^T Y, both MN-major
-      constexpr uint32_t id_kt = umma_idesc_bf16(128, 64, false, true);    // [q x d] = dS K, A K-major, B MN-major
-      const uint32_t aq = smem_u32(sQ), ado = smem_u32(sDO), ak = smem_u32(sK), av = smem_u32(sV), ap = smem_u32(sP);
-      mbar_wait(in_full, 0);
-      tc_fence_after();
-#pragma unroll
-      for (int kk = 0; kk < HD / 16; ++kk)   // S = Q K^T
-        umma_bf16_ss(tS, umma_smem_desc_sw128(aq + kk * 32, 16, 1024), umma_smem_desc_sw128(ak + kk * 32, 16, 1024), id_kk,
-                     kk > 0);
-#pragma unroll
-      for (int kk = 0; kk < HD / 16; ++kk)   // dP = dO V^T
-        umma_bf16_ss(tDP, umma_smem_desc_sw128(ado + kk * 32, 16, 1024), umma_smem_desc_sw128(av + kk * 32, 16, 1024), id_kk,
-                     kk > 0);
-      umma_commit(sdp_ready);
-      mbar_wait(pd_ready, 0);
-      tc_fence_after();
-#pragma unroll
-      for (int kk = 0; kk < TILE / 16; ++kk)   // dV = P~^T dO   (reduction over the query rows) -> overwrites S[0,64)
-        umma_bf16_ss(tDV, umma_smem_desc_sw128(ap + kk * 2048, 16384, 1024), umma_smem_desc_sw128(ado + kk * 2048, 8192, 1024),
-                     id_tt, kk > 0);
-      umma_commit(dv_done);
-      mbar_wait(ds_ready, 0);
-      tc_fence_after();
-#pragma unroll
-      for (int kk = 0; kk < TILE / 16; ++kk)   // dK = dS^T Q -> S[64,128)
-        umma_bf16_ss(tDK, umma_smem_desc_sw128(ap + kk * 2048, 16384, 1024), umma_smem_desc_sw128(aq + kk * 2048, 8192, 1024),
-                     id_tt, kk > 0);
-#pragma unroll
-      for (int kk = 0; kk < TILE / 16; ++kk)   // dQ = dS K (reduction over the keys) -> dP[0,64)
-        umma_bf16_ss(tDQ, umma_smem_desc_sw128(ap + (kk >> 2) * 16384 + (kk & 3) * 32, 16, 1024),
-                     umma_smem_desc_sw128(ak + kk * 2048, 8192, 1024), id_kt, kk > 0);
-      umma_commit(fin);
-    }
-  } else {
-    const int r = (warp & 3) * 32 + lane;        // query row inside the tile == TMEM lane
-    const int ch = warp >> 2;                    // which 64-column half this thread handles
-    const uint32_t lane_base = uint32_t((warp & 3) * 32) << 16;
-    const float c_scale = p.scale * LOG2E;
-    const int q = r;
-    const bool q_ok = q < p.S;
-    const float lse2 = q_ok ? p.lse[(size_t)bh * p.S + q] * LOG2E : 0.f;
-    // delta = <dO, O> of the row, computed here instead of in a separate pass: this thread's 32 columns of O come
-    // from global memory (issued before any wait), dO from the tile TMA already brought in
-    uint4 ov[4];
-#pragma unroll
-    for (int g = 0; g < 4; ++g)
-      ov[g] = q_ok ? __ldg(reinterpret_cast<const uint4*>(p.ctx + (size_t)(row0 + q) * p.H + head * HD + ch * 32 + g * 8))
-                   : make_uint4(0, 0, 0, 0);
-    mbar_wait(in_full, 0);
-    float part = 0.f;
-#pragma unroll
-    for (int g = 0; g < 4; ++g) {
-      const uint4 dv = *reinterpret_cast<const uint4*>(sDO + r * 128 + (((ch * 4 + g) ^ (r & 7)) << 4));
-      const uint32_t a[4] = {ov[g].x, ov[g].y, ov[g].z, ov[g].w}, d[4] = {dv.x, dv.y, dv.z, dv.w};
-#pragma unroll
-      for (int t = 0; t < 4; ++t) {
-        const float2 x = unpack_bf16(a[t]), y = unpack_bf16(d[t]);
-        part += x.x * y.x + x.y * y.y;
-      }
-    }
-    xch[ch * 128 + r] = part;
-    asm volatile("bar.sync 1, 256;" ::: "memory");
-    const float dlt = q_ok ? xch[r] + xch[128 + r] : 0.f;
-    const uint64_t erow = ((uint64_t)bh * p.S + (uint64_t)q) * (uint64_t)p.S;
-    uint32_t dsp[32];                            // this thread's 64 dS values, packed bf16
-    const float qscale8 = p.f8.q ? p.f8.meta[1] : 0.f;
-    float amax8 = 0.f;
-    mbar_wait(sdp_ready, 0);
-    tc_fence_after();
-#pragma unroll
-    for (int sc = 0; sc < 4; ++sc) {             // 16-column sub-chunks of this thread's key half
-      const int c16 = ch * 4 + sc;
-      uint32_t sv[16], dv[16];
-      tmem_ld_32x16(tS + lane_base + c16 * 16, sv);
-      tmem_ld_32x16(tDP + lane_base + c16 * 16, dv);
-      tmem_ld_wait();
-      const int k0 = c16 * 16;
-#pragma unroll
-      for (int g = 0; g < 2; ++g) {
-        Keep8 keep = Keep8::all();
-        if (p.thresh16 != 0) keep = dropout_keep8(seed, p.stream, (erow + (uint64_t)(k0 + g * 8)) >> 3, p.thresh16);
-        float pd[8], ds[8];
-#pragma unroll
-        for (int t = 0; t < 8; ++t) {
-          const int key = k0 + g * 8 + t;
-          const bool ok = q_ok && key < seqlen;
-          const float pr = ok ? ex2_approx(fmaf(__uint_as_float(sv[g * 8 + t]), c_scale, -lse2)) : 0.f;
-          const bool kp = keep[t];
-          const float dp = kp ? __uint_as_float(dv[g * 8 + t]) * p.inv_keep : 0.f;
-          pd[t] = kp ? pr * p.inv_keep : 0.f;
-          ds[t] = pr * (dp - dlt) * p.scale;
-        }
-        *reinterpret_cast<uint4*>(sP + p_chunk_offset(r, c16 * 2 + g)) =
-            make_uint4(pack_bf16(pd[0], pd[1]), pack_bf16(pd[2], pd[3]), pack_bf16(pd[4], pd[5]), pack_bf16(pd[6], pd[7]));
-#pragma unroll
-        for (int t = 0; t < 4; ++t) dsp[(sc * 2 + g) * 4 + t] = pack_bf16(ds[2 * t], ds[2 * t + 1]);
-      }
-    }
-    fence_proxy_async();
-    tc_fence_before();                           // S / dP reads retired before dV may overwrite S
-    mbar_arrive(pd_ready);
-    mbar_wait(dv_done, 0);                       // the tensor core no longer reads P~
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-      *reinterpret_cast<uint4*>(sP + p_chunk_offset(r, ch * 8 + i)) =
-          make_uint4(dsp[i * 4], dsp[i * 4 + 1], dsp[i * 4 + 2], dsp[i * 4 + 3]);
-    fence_proxy_async();
-    mbar_arrive(ds_ready);
-    mbar_wait(fin, 0);
-    tc_fence_after();
-    // epilogue: column half 0 writes dQ[:, 0:32], dK; half 1 writes dQ[:, 32:64], dV
-    {
-      uint32_t v[32];
-      tmem_ld_32x32(tDQ + lane_base + ch * 32, v);
-      tmem_ld_wait();
-      if (q_ok) {
-        __nv_bfloat16* dq = p.dqkv + (size_t)(row0 + q) * 3 * p.H + head * HD + ch * 32;
-#pragma unroll
-        for (int g = 0; g < 4; ++g)
-          *reinterpret_cast<uint4*>(dq + g * 8) = make_uint4(
-              pack_bf16(__uint_as_float(v[g * 8]), __uint_as_float(v[g * 8 + 1])),
-              pack_bf16(__uint_as_float(v[g * 8 + 2]), __uint_as_float(v[g * 8 + 3])),
-              pack_bf16(__uint_as_float(v[g * 8 + 4]), __uint_as_float(v[g * 8 + 5])),
-              pack_bf16(__uint_as_float(v[g * 8 + 6]), __uint_as_float(v[g * 8 + 7])));
-        if (p.f8.q) emit_fp8_row<4>(p.f8, (size_t)(row0 + q) * 3 * p.H + head * HD + ch * 32, v, 1.f, qscale8, amax8);
-      }
-    }
-    const int key = r;
-    const uint32_t src = ch == 0 ? tDK : tDV;
-#pragma unroll 1
-    for (int c = 0; c < 2; ++c) {
-      uint32_t v[32];
-      tmem_ld_32x32(src + lane_base + c * 32, v);
-      tmem_ld_wait();
-      if (key < p.S) {
-        __nv_bfloat16* dst = p.dqkv + (size_t)(row0 + key) * 3 * p.H + (ch + 1) * p.H + head * HD + c * 32;
-#pragma unroll
-        for (int g = 0; g < 4; ++g)
-          *reinterpret_cast<uint4*>(dst + g * 8) = make_uint4(
-              pack_bf16(__uint_as_float(v[g * 8]), __uint_as_float(v[g * 8 + 1])),
-              pack_bf16(__uint_as_float(v[g * 8 + 2]), __uint_as_float(v[g * 8 + 3])),
-              pack_bf16(__uint_as_float(v[g * 8 + 4]), __uint_as_float(v[g * 8 + 5])),
-              pack_bf16(__uint_as_float(v[g * 8 + 6]), __uint_as_float(v[g * 8 + 7])));
-        if (p.f8.q)
-          emit_fp8_row<4>(p.f8, (size_t)(row0 + key) * 3 * p.H + (ch + 1) * p.H + head * HD + c * 32, v, 1.f, qscale8, amax8);
-      }
-    }
-    if (p.f8.q) fp8_amax_commit(p.f8, amax8);
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 8) {
-    tc_fence_after();
-    tmem_dealloc(tmem, 256);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Round-2 backward, S <= 128: one THREAD per query row (scores, dP, lse and delta of a row never leave the thread),
-// persistent CTAs.  Same MMA chain as attn_bwd_single_kernel (S = Q K^T, dP = dO V^T -> P~ -> dV = P~^T dO;
-// dS -> dK = dS^T Q, dQ = dS K; dV / dK / dQ overwrite the consumed S / dP accumulators; one 32 KB buffer carries P~
-// and then dS), but
-//   * 12 instead of ~33 instructions per score element: 1 / keep_prob in the exponent, dS = p' * select(keep,
-//     dP * scale + c, c) with the row constants folded, hoisted Philox keys, in-place 16-bit keep compares, no
-//     shared-memory exchange for delta = <dO, O> (one thread computes the whole row dot product);
-//   * the loop over (batch, head) items keeps TMEM / barriers alive, V of the next item streams in under the
-//     softmax-gradient math and Q / K / dO under the epilogue stores.
-// 96 KB, 256 TMEM columns, 160 threads -> two CTAs per SM.
-// ------------------------------------------------------------------------------------------------
+// P~ and dS of 16 score columns of one row, packed bf16: p' = 2^(s c + off) = P / keep_prob, u = dP a + bq
 template <bool FULL, bool DROP>
 __device__ __forceinline__ void dsoftmax_chunk16(const uint32_t (&sv)[16], const uint32_t (&dv)[16], uint32_t (&pw)[8],
                                                  uint32_t (&dw)[8], float c_scale, float off, float a, float bq, int nvalid,
@@ -1747,241 +889,6 @@ __device__ __forceinline__ void dsoftmax_chunk16(const uint32_t (&sv)[16], const
     }
   }
 }
-
-__global__ void __launch_bounds__(ATT_ROW_THREADS, 2)
-attn_bwd_row_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_do,
-                    const AttnArgs p, const int n_items) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sK = smem;                      // 16 KB each
-  uint8_t* sV = smem + 16384;
-  uint8_t* sQ = smem + 16384 * 2;
-  uint8_t* sDO = smem + 16384 * 3;
-  uint8_t* sP = smem + 16384 * 4;          // 32 KB: P~, later dS
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 16384 * 6);
-  uint64_t* qkd_full = bars;               // Q, K, dO of an item landed
-  uint64_t* v_full = bars + 1;             // V landed
-  uint64_t* sdp_ready = bars + 2;          // S and dP complete (V is free)
-  uint64_t* pd_ready = bars + 3;           // 128 threads: P~ is in shared memory, S / dP consumed
-  uint64_t* dv_done = bars + 4;            // dV MMA retired: the buffer may be overwritten with dS
-  uint64_t* ds_ready = bars + 5;           // 128 threads: dS is in shared memory
-  uint64_t* fin = bars + 6;                // dK, dQ complete (Q, K, dO, the buffer are free)
-  uint64_t* acc_read = bars + 7;           // 128 threads: dQ / dK / dV read out of tensor memory
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 8);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 128) {
-    tma_prefetch_desc(&tmap_qkv);
-    tma_prefetch_desc(&tmap_do);
-    mbar_init(qkd_full, 1);
-    mbar_init(v_full, 1);
-    mbar_init(sdp_ready, 1);
-    mbar_init(pd_ready, 128);
-    mbar_init(dv_done, 1);
-    mbar_init(ds_ready, 128);
-    mbar_init(fin, 1);
-    mbar_init(acc_read, 128);
-    fence_barrier_init();
-  }
-  if (warp == 4) tmem_alloc(tmem_slot, 256);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const uint32_t tS = tmem, tDP = tmem + 128, tDV = tmem, tDK = tmem + 64, tDQ = tmem + 128;
-
-  if (warp == 4) {
-    if (lane == 0) {
-      constexpr uint32_t id_kk = umma_idesc_bf16(128, 128, false, false);  // [q x keys], both K-major
-      constexpr uint32_t id_tt = umma_idesc_bf16(128, 64, true, true);     // [keys x d] = X^T Y, both MN-major
-      constexpr uint32_t id_kt = umma_idesc_bf16(128, 64, false, true);    // [q x d] = dS K, A K-major, B MN-major
-      const uint32_t aq = smem_u32(sQ), ado = smem_u32(sDO), ak = smem_u32(sK), av = smem_u32(sV), ap = smem_u32(sP);
-      auto load_qkd = [&](int item) {
-        const int b = item / p.h, head = item - b * p.h;
-        mbar_arrive_expect_tx(qkd_full, 49152);
-        tma_load_2d(sK, &tmap_qkv, qkd_full, p.H + head * HD, b * p.S);
-        tma_load_2d(sQ, &tmap_qkv, qkd_full, head * HD, b * p.S);
-        tma_load_2d(sDO, &tmap_do, qkd_full, head * HD, b * p.S);
-      };
-      auto load_v = [&](int item) {
-        const int b = item / p.h, head = item - b * p.h;
-        mbar_arrive_expect_tx(v_full, 16384);
-        tma_load_2d(sV, &tmap_qkv, v_full, 2 * p.H + head * HD, b * p.S);
-      };
-      int item = blockIdx.x;
-      if (item < n_items) { load_qkd(item); load_v(item); }
-      for (uint32_t g = 0; item < n_items; item += gridDim.x, ++g) {
-        const int nitem = item + gridDim.x;
-        const uint32_t ph = g & 1;
-        if (g > 0) mbar_wait(acc_read, (g - 1) & 1);           // previous dQ / dK / dV drained
-        mbar_wait(qkd_full, ph);
-        mbar_wait(v_full, ph);
-        tc_fence_after();
-#pragma unroll
-        for (int kk = 0; kk < HD / 16; ++kk)   // S = Q K^T
-          umma_bf16_ss(tS, umma_smem_desc_sw128(aq + kk * 32, 16, 1024), umma_smem_desc_sw128(ak + kk * 32, 16, 1024), id_kk, kk > 0);
-#pragma unroll
-        for (int kk = 0; kk < HD / 16; ++kk)   // dP = dO V^T
-          umma_bf16_ss(tDP, umma_smem_desc_sw128(ado + kk * 32, 16, 1024), umma_smem_desc_sw128(av + kk * 32, 16, 1024), id_kk, kk > 0);
-        umma_commit(sdp_ready);
-        mbar_wait(sdp_ready, ph);                              // V is free: the next one streams in under the math
-        if (nitem < n_items) load_v(nitem);
-        mbar_wait(pd_ready, ph);
-        tc_fence_after();
-#pragma unroll
-        for (int kk = 0; kk < TILE / 16; ++kk)   // dV = P~^T dO -> S[0,64)
-          umma_bf16_ss(tDV, umma_smem_desc_sw128(ap + kk * 2048, 16384, 1024), umma_smem_desc_sw128(ado + kk * 2048, 8192, 1024), id_tt, kk > 0);
-        umma_commit(dv_done);
-        mbar_wait(ds_ready, ph);
-        tc_fence_after();
-#pragma unroll
-        for (int kk = 0; kk < TILE / 16; ++kk)   // dK = dS^T Q -> S[64,128)
-          umma_bf16_ss(tDK, umma_smem_desc_sw128(ap + kk * 2048, 16384, 1024), umma_smem_desc_sw128(aq + kk * 2048, 8192, 1024), id_tt, kk > 0);
-#pragma unroll
-        for (int kk = 0; kk < TILE / 16; ++kk)   // dQ = dS K -> dP[0,64)
-          umma_bf16_ss(tDQ, umma_smem_desc_sw128(ap + (kk >> 2) * 16384 + (kk & 3) * 32, 16, 1024),
-                       umma_smem_desc_sw128(ak + kk * 2048, 8192, 1024), id_kt, kk > 0);
-        umma_commit(fin);
-        mbar_wait(fin, ph);                                    // Q, K, dO free: next item streams in under the epilogue
-        if (nitem < n_items) load_qkd(nitem);
-      }
-    }
-  } else {
-    const int r = warp * 32 + lane;                            // query row == key row of the epilogue == TMEM lane
-    const uint32_t lane_base = uint32_t(warp * 32) << 16;
-    const float c_scale = p.scale * LOG2E;
-    const bool drop = p.thresh16 != 0;
-    const float lk = drop ? log2f(p.inv_keep) : 0.f;
-    const uint32_t T = p.thresh16 << 16;
-    const PhiloxKeys keys = philox_keys(drop ? p.seed.value() : 0ull);
-    const bool row_ok = r < p.S;
-    const float qscale8 = p.f8.q ? p.f8.meta[1] : 0.f;
-    float amax8 = 0.f;
-    uint32_t g = 0;
-    for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++g) {
-      const uint32_t ph = g & 1;
-      const int b = item / p.h, head = item - b * p.h;
-      const int seqlen = min(__ldg(p.seqlens + b), p.S);
-      const size_t tok = (size_t)b * p.S + r;
-      // this row's O (global, issued before any wait) and log-sum-exp
-      uint4 ov[8];
-#pragma unroll
-      for (int c = 0; c < 8; ++c)
-        ov[c] = row_ok ? __ldg(reinterpret_cast<const uint4*>(p.ctx + tok * p.H + head * HD + c * 8)) : make_uint4(0, 0, 0, 0);
-      const float lse2 = row_ok ? __ldg(p.lse + (size_t)item * p.S + r) * LOG2E : 0.f;
-      mbar_wait(qkd_full, ph);
-      float dlt = 0.f;                                         // delta = <dO, O> of the row
-#pragma unroll
-      for (int c = 0; c < 8; ++c) {
-        const uint4 dv = *reinterpret_cast<const uint4*>(sDO + r * 128 + ((c ^ (r & 7)) << 4));
-        const uint32_t aw[4] = {ov[c].x, ov[c].y, ov[c].z, ov[c].w}, dw[4] = {dv.x, dv.y, dv.z, dv.w};
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const float2 x = unpack_bf16(aw[t]), y = unpack_bf16(dw[t]);
-          dlt = fmaf(x.x, y.x, fmaf(x.y, y.y, dlt));
-        }
-      }
-      const float off = lk - lse2;                             // p' = 2^(s c + off) = P / keep_prob
-      const float a = p.scale;                                 // dS = p' * (keep ? dP * scale + bq : bq)
-      const float bq = -dlt * p.scale / p.inv_keep;
-      const int kvalid = row_ok ? seqlen : 0;                  // rows beyond the sequence contribute nothing
-      const uint64_t e8row = (((uint64_t)item * p.S + (uint64_t)r) * (uint64_t)p.S) >> 3;
-      uint32_t dsp[64];                                        // this row's 128 dS values, packed bf16
-      mbar_wait(sdp_ready, ph);
-      tc_fence_after();
-      {
-        uint32_t sv[2][16], dv[2][16];
-        tmem_ld_32x16(tS + lane_base, sv[0]);
-        tmem_ld_32x16(tDP + lane_base, dv[0]);
-#pragma unroll
-        for (int c = 0; c < 8; ++c) {                          // 16-column chunks, the next one in flight
-          tmem_ld_wait();
-          if (c + 1 < 8) {
-            tmem_ld_32x16(tS + lane_base + (c + 1) * 16, sv[(c + 1) & 1]);
-            tmem_ld_32x16(tDP + lane_base + (c + 1) * 16, dv[(c + 1) & 1]);
-          }
-          const int nv = kvalid - c * 16;
-          uint32_t pw[8];
-          uint32_t (&dw)[8] = *reinterpret_cast<uint32_t (*)[8]>(&dsp[c * 8]);
-          const uint64_t e8 = e8row + (uint64_t)(2 * c);
-          if (nv >= 16) {
-            if (drop) dsoftmax_chunk16<true, true>(sv[c & 1], dv[c & 1], pw, dw, c_scale, off, a, bq, 16, keys, e8, p.stream, T);
-            else dsoftmax_chunk16<true, false>(sv[c & 1], dv[c & 1], pw, dw, c_scale, off, a, bq, 16, keys, e8, p.stream, T);
-          } else if (nv > 0) {
-            if (drop) dsoftmax_chunk16<false, true>(sv[c & 1], dv[c & 1], pw, dw, c_scale, off, a, bq, nv, keys, e8, p.stream, T);
-            else dsoftmax_chunk16<false, false>(sv[c & 1], dv[c & 1], pw, dw, c_scale, off, a, bq, nv, keys, e8, p.stream, T);
-          } else {
-#pragma unroll
-            for (int t = 0; t < 8; ++t) { pw[t] = 0u; dw[t] = 0u; }
-          }
-          *reinterpret_cast<uint4*>(sP + p_chunk_offset(r, c * 2)) = make_uint4(pw[0], pw[1], pw[2], pw[3]);
-          *reinterpret_cast<uint4*>(sP + p_chunk_offset(r, c * 2 + 1)) = make_uint4(pw[4], pw[5], pw[6], pw[7]);
-        }
-      }
-      fence_proxy_async();
-      tc_fence_before();                                       // S / dP reads retired before dV may overwrite S
-      mbar_arrive(pd_ready);
-      mbar_wait(dv_done, ph);                                  // the tensor core no longer reads P~
-#pragma unroll
-      for (int i = 0; i < 16; ++i)
-        *reinterpret_cast<uint4*>(sP + p_chunk_offset(r, i)) = make_uint4(dsp[i * 4], dsp[i * 4 + 1], dsp[i * 4 + 2], dsp[i * 4 + 3]);
-      fence_proxy_async();
-      mbar_arrive(ds_ready);
-      mbar_wait(fin, ph);
-      tc_fence_after();
-      // ---- epilogue: this thread's rows of dQ (query r), dK and dV (key r)
-      __nv_bfloat16* drow = p.dqkv + tok * 3 * p.H + head * HD;
-#pragma unroll
-      for (int w = 0; w < 3; ++w) {
-        const uint32_t src = w == 0 ? tDQ : (w == 1 ? tDK : tDV);
-#pragma unroll
-        for (int hh = 0; hh < 2; ++hh) {
-          uint32_t v[32];
-          tmem_ld_32x32(src + lane_base + hh * 32, v);
-          tmem_ld_wait();
-          if (w == 2 && hh == 1) {                             // accumulators drained: the next item's MMAs may go
-            tc_fence_before();
-            mbar_arrive(acc_read);
-          }
-          if (row_ok) {
-            __nv_bfloat16* dst = drow + w * p.H + hh * 32;
-#pragma unroll
-            for (int gq = 0; gq < 4; ++gq)
-              *reinterpret_cast<uint4*>(dst + gq * 8) = make_uint4(
-                  pack_bf16(__uint_as_float(v[gq * 8]), __uint_as_float(v[gq * 8 + 1])),
-                  pack_bf16(__uint_as_float(v[gq * 8 + 2]), __uint_as_float(v[gq * 8 + 3])),
-                  pack_bf16(__uint_as_float(v[gq * 8 + 4]), __uint_as_float(v[gq * 8 + 5])),
-                  pack_bf16(__uint_as_float(v[gq * 8 + 6]), __uint_as_float(v[gq * 8 + 7])));
-            if (p.f8.q) emit_fp8_row<4>(p.f8, tok * 3 * p.H + (size_t)(w * p.H + head * HD + hh * 32), v, 1.f, qscale8, amax8);
-          }
-        }
-      }
-    }
-    if (p.f8.q) fp8_amax_commit(p.f8, amax8);
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 4) {
-    tc_fence_after();
-    tmem_dealloc(tmem, 256);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Backward, S <= 128, second layout (default): TWO threads per query row (64 key columns each, 8 math warps) with the
-// lean per-element math of attn_bwd_row_kernel, persistent CTAs, and dS PARKED IN TENSOR MEMORY.
-// ncu on the one-thread-per-row kernel: 19 % issue utilisation, long_scoreboard / barrier waits dominate -- four math
-// warps per CTA cannot hide the dependent MMA -> math -> MMA -> math -> MMA chain and the global loads of O / lse at
-// the head of an item, and the 64 registers of packed dS forced full unrolling (8720 instructions, instruction-cache
-// misses).  Here
-//   * every 16-column chunk's dS (8 packed words) is written back with tcgen05.st into the upper half of the thread's
-//     own, already consumed dP columns (chunks run right to left, so the target columns are always behind the read
-//     pointer) and copied to shared memory once the dV MMA has released the P~ buffer: no register array survives the
-//     chunk loop, which therefore stays rolled (small code, 16-byte shared-memory stores);
-//   * the O half-row and log-sum-exp of the NEXT item are fetched while this item waits for its last MMAs;
-//   * delta = <dO, O>: each thread of a row computes half, one shared-memory exchange + named barrier per item.
-// 96 KB, 256 TMEM columns, 288 threads -> two CTAs per SM (16 math warps per SM).
-// ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void tmem_st_32x8(uint32_t taddr, const uint32_t (&v)[8]) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(v[0]),
                "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]) : "memory");
@@ -2257,6 +1164,17 @@ static void fill_args(AttnArgs& a, int B, int S, int h, int d, const int* seqlen
   a.ctx = nullptr; a.lse = nullptr; a.delta = nullptr; a.dqkv = nullptr; a.dq_acc = nullptr;
 }
 
+// multiprocessor count of the current device: the persistent kernels launch a fixed number of CTAs per SM
+static int sm_count() {
+  static int sms = 0;
+  if (sms == 0) {
+    int dev;
+    B200_CUDA_CHECK(cudaGetDevice(&dev));
+    B200_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  }
+  return sms;
+}
+
 void attention_fwd(const void* qkv, const int* seqlens, void* ctx, float* lse, int B, int S, int h, int d,
                    float scale, Seed seed, unsigned int stream, float p_drop, Fp8Out f8, cudaStream_t st) {
   AttnArgs a;
@@ -2264,56 +1182,21 @@ void attention_fwd(const void* qkv, const int* seqlens, void* ctx, float* lse, i
   a.ctx = (__nv_bfloat16*)ctx; a.lse = lse; a.f8 = f8;
   const int H = h * d;
   CUtensorMap tm = make_tmap_2d_bf16(qkv, 3 * H, (uint64_t)B * S, 3 * H, 64, TILE);
-  dim3 grid((S + TILE - 1) / TILE, B * h);
-  if (attn_row_enabled()) {                      // round-2 kernels: thread per query row, P in TMEM, persistent CTAs
-    static int sms = 0;
-    if (sms == 0) {
-      int dev;
-      B200_CUDA_CHECK(cudaGetDevice(&dev));
-      B200_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    }
-    const int nqb = (S + TILE - 1) / TILE, n_items = nqb * B * h;
-    if (S <= TILE) {
-      constexpr int SMEMR = 16384 * 3 + 1024 + 128;
-      static bool once = false;
-      if (!once) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd_row_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEMR)); once = true; }
-      const int g = n_items < sms * 4 ? n_items : sms * 4;
-      launch_pdl(attn_fwd_row_kernel, dim3(g), dim3(ATT_ROW_THREADS), SMEMR, st, tm, a, n_items);
-    } else {
-      constexpr int SMEMS = 16384 * 5 + 1024 + 256;
-      static bool once = false;
-      if (!once) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEMS)); once = true; }
-      const int g = n_items < sms * 2 ? n_items : sms * 2;
-      attn_fwd_stream_kernel<<<g, ATT_STREAM_THREADS, SMEMS, st>>>(tm, a, n_items, nqb);
-    }
-    return;
-  }
-  static const bool single_ok = []() { const char* e = getenv("B200_ATTN_FWD_SINGLE"); return !(e && e[0] == '0'); }();
-  if (S <= TILE && single_ok) {
-    constexpr int SMEM1 = 16384 * 3 + 1024 + 64 + 2048;
-    static bool once1 = false;
-    if (!once1) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd_single_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM1)); once1 = true; }
-    attn_fwd_single_kernel<<<grid, ATT_BWD_THREADS, SMEM1, st>>>(tm, a);
-  } else if (S <= TILE) {
-    constexpr int SMEM = 16384 * 5 + 1024 + 128 + 3200;
+  const int sms = sm_count();
+  const int nqb = (S + TILE - 1) / TILE, n_items = nqb * B * h;
+  if (S <= TILE) {
+    constexpr int SMEMR = 16384 * 3 + 1024 + 128;
     static bool once = false;
-    if (!once) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM)); once = true; }
-    attn_fwd_kernel<1><<<grid, ATT_BWD_THREADS, SMEM, st>>>(tm, a);
+    if (!once) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd_row_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEMR)); once = true; }
+    const int g = n_items < sms * 4 ? n_items : sms * 4;
+    launch_pdl(attn_fwd_row_kernel, dim3(g), dim3(ATT_ROW_THREADS), SMEMR, st, tm, a, n_items);
   } else {
-    constexpr int SMEM = 16384 * 6 + 1024 + 128 + 3200;
+    constexpr int SMEMS = 16384 * 5 + 1024 + 256;
     static bool once = false;
-    if (!once) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM)); once = true; }
-    attn_fwd_kernel<2><<<grid, ATT_BWD_THREADS, SMEM, st>>>(tm, a);
+    if (!once) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEMS)); once = true; }
+    const int g = n_items < sms * 2 ? n_items : sms * 2;
+    attn_fwd_stream_kernel<<<g, ATT_STREAM_THREADS, SMEMS, st>>>(tm, a, n_items, nqb);
   }
-}
-
-// -1: follow B200_ATTN_BWD_PIPE (default on), 0 / 1: forced by the caller
-static int g_bwd_pipe = -1;
-void attention_set_options(int bwd_pipe, int row_kernels) { g_bwd_pipe = bwd_pipe; g_attn_row = row_kernels; }
-static bool attn_bwd_pipe_enabled() {
-  if (g_bwd_pipe >= 0) return g_bwd_pipe != 0;
-  static const bool env_on = []() { const char* e = getenv("B200_ATTN_BWD_PIPE"); return !(e && e[0] == '0'); }();
-  return env_on;    // default on since round 2: 188 vs 208 us at 16 x 512 (profiles/attn_bench_r2_pipe.jsonl)
 }
 
 void attention_bwd(const void* qkv, const int* seqlens, const void* ctx, const void* dctx, const float* lse,
@@ -2325,89 +1208,30 @@ void attention_bwd(const void* qkv, const int* seqlens, const void* ctx, const v
   const int H = h * d;
   a.lse = const_cast<float*>(lse); a.delta = delta_ws; a.dqkv = (__nv_bfloat16*)dqkv; a.dq_acc = dq_acc;
   a.ctx = (__nv_bfloat16*)const_cast<void*>(ctx);
-  const int nkb = (S + TILE - 1) / TILE;
-  static const bool single_ok = []() { const char* e = getenv("B200_ATTN_BWD_SINGLE"); return !(e && e[0] == '0'); }();
-  if (!(nkb == 1 && single_ok)) {               // the single-block kernel computes delta itself
-    const long long groups = (long long)B * S * h;
-    attn_delta_kernel<<<(unsigned)((groups * 8 + 255) / 256), 256, 0, st>>>((const __nv_bfloat16*)ctx,
-                                                                         (const __nv_bfloat16*)dctx, delta_ws, B, S, h, H);
-  }
-  if (nkb > 1) {
-    if (dq_acc == nullptr) { fprintf(stderr, "[b200] attention_bwd needs a dq accumulation buffer when S > 128\n"); abort(); }
-    B200_CUDA_CHECK(cudaMemsetAsync(dq_acc, 0, sizeof(float) * (size_t)B * S * H, st));
-  }
   CUtensorMap tq = make_tmap_2d_bf16(qkv, 3 * H, (uint64_t)B * S, 3 * H, 64, TILE);
   CUtensorMap td = make_tmap_2d_bf16(dctx, H, (uint64_t)B * S, H, 64, TILE);
-  constexpr int SMEM = 16384 * 10 + 1024 + 128;
-  static bool once = false;
-  if (!once) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM)); once = true; }
-  dim3 grid(nkb, B * h);
-  // the thread-per-row backward is correct but, with only four math warps per CTA, latency bound (ncu: 19 % issue
-  // utilisation, 103 vs 93 us): opt-in until it has the two-threads-per-row / TMEM-parked dS layout (NOTES.md)
-  static const int bwd_row = []() { const char* e = getenv("B200_ATTN_BWD_ROW"); return e ? atoi(e) : 2; }();
-  if (nkb == 1 && single_ok && attn_row_enabled() && bwd_row == 2) {   // two threads per row, dS parked in TMEM, persistent
-    static int sms = 0;
-    if (sms == 0) {
-      int dev;
-      B200_CUDA_CHECK(cudaGetDevice(&dev));
-      B200_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    }
+  if (S <= TILE) {                               // one key block; the kernel computes delta itself
     constexpr int SMEM2 = 16384 * 6 + 1024 + 128 + 2048;
-    static bool once2 = false;
-    if (!once2) {
-      B200_CUDA_CHECK(cudaFuncSetAttribute(attn_bwd_row2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM2));
-      once2 = true;
-    }
-    const int n_items = B * h;
+    static bool once = false;
+    if (!once) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_bwd_row2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM2)); once = true; }
+    const int n_items = B * h, sms = sm_count();
     const int g = n_items < sms * 2 ? n_items : sms * 2;
     launch_pdl(attn_bwd_row2_kernel, dim3(g), dim3(ATT_BWD_THREADS), SMEM2, st, tq, td, a, n_items);
     return;
   }
-  if (nkb == 1 && single_ok && attn_row_enabled() && bwd_row == 1) {       // round-2 kernel: thread per query row, persistent CTAs
-    static int sms = 0;
-    if (sms == 0) {
-      int dev;
-      B200_CUDA_CHECK(cudaGetDevice(&dev));
-      B200_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    }
-    constexpr int SMEMR = 16384 * 6 + 1024 + 128;
-    static bool oncer = false;
-    if (!oncer) {
-      B200_CUDA_CHECK(cudaFuncSetAttribute(attn_bwd_row_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEMR));
-      oncer = true;
-    }
-    const int n_items = B * h;
-    const int g = n_items < sms * 2 ? n_items : sms * 2;
-    attn_bwd_row_kernel<<<g, ATT_ROW_THREADS, SMEMR, st>>>(tq, td, a, n_items);
-    return;
-  }
-  if (nkb == 1 && single_ok) {                 // S <= 128: the two-CTAs-per-SM variant
-    constexpr int SMEM1 = 16384 * 6 + 1024 + 128 + 1024;
-    static bool once1 = false;
-    if (!once1) {
-      B200_CUDA_CHECK(cudaFuncSetAttribute(attn_bwd_single_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM1));
-      once1 = true;
-    }
-    attn_bwd_single_kernel<<<grid, ATT_BWD_THREADS, SMEM1, st>>>(tq, td, a);
-    return;
-  }
-  if (nkb > 1 && attn_bwd_pipe_enabled()) {      // software-pipelined variant (opt-in)
-    constexpr int SMEMP = 16384 * 12 + 1024 + 128;
-    static bool oncep = false;
-    if (!oncep) {
-      B200_CUDA_CHECK(cudaFuncSetAttribute(attn_bwd_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEMP));
-      oncep = true;
-    }
-    attn_bwd_pipe_kernel<<<grid, ATT_BWD16_THREADS, SMEMP, st>>>(tq, td, a);
-  } else {
-    attn_bwd_kernel<<<grid, ATT_BWD16_THREADS, SMEM, st>>>(tq, td, a);
-  }
-  if (nkb > 1) {
-    const long long work = (long long)B * S * (H / 8);
-    int g = (int)((work + 255) / 256);
-    if (g > 148 * 16) g = 148 * 16;
-    attn_dq_convert_kernel<<<g, 256, 0, st>>>(dq_acc, (__nv_bfloat16*)dqkv, (long long)B * S, H, a.f8);
-  }
+  if (dq_acc == nullptr) { fprintf(stderr, "[b200] attention_bwd needs a dq accumulation buffer when S > 128\n"); abort(); }
+  const long long groups = (long long)B * S * h;
+  attn_delta_kernel<<<(unsigned)((groups * 8 + 255) / 256), 256, 0, st>>>((const __nv_bfloat16*)ctx,
+                                                                       (const __nv_bfloat16*)dctx, delta_ws, B, S, h, H);
+  B200_CUDA_CHECK(cudaMemsetAsync(dq_acc, 0, sizeof(float) * (size_t)B * S * H, st));
+  constexpr int SMEMP = 16384 * 12 + 1024 + 128;
+  static bool once = false;
+  if (!once) { B200_CUDA_CHECK(cudaFuncSetAttribute(attn_bwd_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEMP)); once = true; }
+  attn_bwd_pipe_kernel<<<dim3((S + TILE - 1) / TILE, B * h), ATT_BWD16_THREADS, SMEMP, st>>>(tq, td, a);
+  const long long work = (long long)B * S * (H / 8);
+  int g = (int)((work + 255) / 256);
+  if (g > 148 * 16) g = 148 * 16;
+  attn_dq_convert_kernel<<<g, 256, 0, st>>>(dq_acc, (__nv_bfloat16*)dqkv, (long long)B * S, H, a.f8);
 }
 
 }  // namespace b200

@@ -560,6 +560,5 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("arena_adam", &arena_adam);
   m.def("attention_fwd", &attention_fwd);
   m.def("attention_bwd", &attention_bwd);
-  m.def("set_attention_options", [](int64_t bwd_pipe, int64_t row) { b200::attention_set_options((int)bwd_pipe, (int)row); });
   m.def("fused_allreduce_lamb", &fused_allreduce_lamb);
 }

@@ -53,7 +53,6 @@ void arena_adam(float* g, float* p, float* m, float* v, void* shadow, const int*
 // attention.cu
 void attention_fwd(const void* qkv, const int* seqlens, void* ctx, float* lse, int B, int S, int h, int d,
                    float scale, Seed seed, unsigned int stream, float p_drop, Fp8Out f8, cudaStream_t st);
-void attention_set_options(int bwd_pipe, int row_kernels);   // each: -1 env default, 0 / 1 force off / on
 void attention_bwd(const void* qkv, const int* seqlens, const void* ctx, const void* dctx, const float* lse,
                    void* dqkv, float* delta_ws, float* dq_acc, int B, int S, int h, int d, float scale,
                    Seed seed, unsigned int stream, float p_drop, Fp8Out f8, cudaStream_t st);

@@ -34,11 +34,4 @@ for B, S in ((96, 128), (16, 512)):
     flops = 4.0 * B * h * S * S * 64
     row = {"B": B, "S": S, "fwd_ms": round(tf, 4), "bwd_ms": round(tb, 4),
            "fwd_tflops": round(flops / tf / 1e9, 1), "bwd_tflops": round(2.5 * flops / tb / 1e9, 1)}
-    if "--old" in sys.argv:                    # the round-1 kernels (two threads per row, serial streaming backward)
-        K.set_attention_options(bwd_pipe=False, row_kernels=False)
-        tf0 = timeit(lambda: K.attention_fwd(qkv, lens, h, p_drop=0.1, seed=1, stream=1))
-        tb0 = timeit(lambda: K.attention_bwd(qkv, lens, ctx, d, lse, h, p_drop=0.1, seed=1, stream=1))
-        K.set_attention_options(None, None)
-        row.update(r1_fwd_ms=round(tf0, 4), r1_bwd_ms=round(tb0, 4), r1_fwd_tflops=round(flops / tf0 / 1e9, 1),
-                   r1_bwd_tflops=round(2.5 * flops / tb0 / 1e9, 1))
     print(json.dumps(row), flush=True)

@@ -14,8 +14,8 @@ from collections import Counter
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SO = os.path.join(ROOT, "bert_pytorch_b200", "ops", "_C.so")
 OUT = os.path.join(ROOT, "profiles", "sass")
-HOT = ["gemm_pair_kernel", "gemm_kernel", "gemm_mx", "attn_fwd_row_kernel", "attn_fwd_stream_kernel", "attn_bwd_row_kernel",
-       "attn_bwd_single_kernel", "attn_bwd_pipe_kernel", "attn_bwd_kernel", "ln_fwd_row_kernel", "ln_bwd3_kernel",
+HOT = ["gemm_pair_kernel", "gemm_kernel", "gemm_mx", "attn_fwd_row_kernel", "attn_fwd_stream_kernel",
+       "attn_bwd_pipe_kernel", "ln_fwd_row_kernel", "ln_bwd3_kernel",
        "fused_allreduce_lamb_kernel", "peer_allreduce_kernel", "lamb_stage1_kernel", "lamb_stage2_kernel",
        "softmax_ce_kernel", "embed_fwd_kernel", "embed_bwd_scatter_kernel", "nsp_head_kernel", "colsum_finalize_kernel",
        "kfac_", "dropout_mask_kernel", "attn_bwd_row2_kernel", "colsum_bf16_kernel"]

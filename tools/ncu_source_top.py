@@ -1,6 +1,6 @@
 """Per-source-line stall-sample totals of one kernel of an Nsight Compute report (compiled with -lineinfo, captured
 with --import-source on), read on the CPU box:
-  python tools/ncu_source_top.py gpurun_out/prof_attn.ncu-rep attn_bwd_row_kernel [N]"""
+  python tools/ncu_source_top.py prof_attn.ncu-rep attn_bwd_row2_kernel [N]"""
 import csv
 import io
 import re
